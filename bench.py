@@ -7,6 +7,7 @@ clip_grad_norm_(params, 1e50) -> Adam step -> MultiplicativeLR step -> loss.item
 
     python bench.py [--gpus N --steps K --warmup W]            our arm (N>1: launched by torch.distributed.run)
     python bench.py --impl reference [...]                      the reference's CPU path (oracle port), rank 0 only
+    python bench.py --dump-outputs DIR [...]                    also write the last timed step's outputs (dump_outputs)
 
 One JSON line on stdout (rank 0).  `value` has the batch resident in HBM when the timed region starts; `e2e`
 goes through the public Module API with the batch in pinned host memory (H2D copy + loss/grad-norm D2H read
@@ -146,6 +147,31 @@ class _stdout_to_stderr:
         return False
 
 
+def dump_outputs(out_dir, last, logits, model, per_tensor=4096, seed=0, max_logits=8 << 20):
+    """Writes what the caller of the timed step holds after its last step, for comparing two builds output for output:
+    loss.npy and grad_norm.npy (float64, the step's two return values), logits.npy (float32, the forward's output, cut
+    to the leading images that fit in `max_logits` elements; eager steps only, the graphed step does not keep it) and
+    weights.npy (float32, the updated weights: up to `per_tensor` elements of every parameter at fixed seeded positions,
+    concatenated in named_parameters() order)."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": np.array(last[0], dtype=np.float64), "grad_norm": np.array(last[1], dtype=np.float64)}
+    if logits is not None:
+        keep = max(1, max_logits // max(1, logits[0].numel()))
+        arrays["logits"] = logits[:keep].float().cpu().numpy()
+    g = torch.Generator().manual_seed(seed)
+    picks = []
+    for _, p in model.named_parameters():
+        flat = p.detach().reshape(-1)
+        if flat.numel() > per_tensor:
+            flat = flat[torch.randint(0, flat.numel(), (per_tensor,), generator=g).sort().values.to(flat.device)]
+        picks.append(flat.float().cpu())
+    arrays["weights"] = torch.cat(picks).numpy()
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 # --------------------------------------------------------------------------------------------------
 # Our arm
 # --------------------------------------------------------------------------------------------------
@@ -195,12 +221,16 @@ def run_ours(args):
         graphed = trainstep.GraphedTrainStep(model, params, lambda preds, x: losses.bce_with_logits_sum_mean(preds, x), x_dev,
                                              lr=spec["lr"], lr_gamma=0.999977)
 
+    last_logits = {}
+
     def step(x):
         if graphed is not None:
             return graphed(x)
         train_model.train()
         opt.zero_grad()
         preds = train_model(x)
+        if args.dump_outputs:
+            last_logits["logits"] = preds.detach()
         loss = losses.bce_with_logits_sum_mean(preds, x)  # the recipes' loss_fn (image_gpt.py:158-162), fused kernel
         loss.backward()
         grad_avg.average_()
@@ -240,6 +270,8 @@ def run_ours(args):
     with ClockSampler(local_rank) as clocks:
         ms_total, last = timed(lambda: step(x_dev), args.steps)
     launches = L.launch_count() - launches0
+    if args.dump_outputs and rank == 0:  # before the passes below move the weights on
+        dump_outputs(args.dump_outputs, last, last_logits.get("logits"), model)
 
     # ---- the same steps again with CUDA events around every GEMM launch, for the roofline line only ----
     gemm_events = []
@@ -416,7 +448,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--sample", action="store_true", help="also time model.sample(n_samples=16)")
     ap.add_argument("--graph", action="store_true", help="replay the whole training step as one CUDA graph (small configs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

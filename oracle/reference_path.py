@@ -14,10 +14,9 @@ come in as a state_dict with the reference's own key names, so a reference check
 
 Pinning: the reference's tests hold no golden vectors for this path (SURVEY.md §8c: "parity
 unpinned" upstream).  The oracle is therefore pinned against outputs of the reference itself, run in
-the build container: `tests/golden/make_golden.py` imports /root/reference, runs seeded tiny configs of
-all four models and the four nn blocks, and commits inputs/outputs under tests/golden/;
-`tests/test_oracle.py` checks this file against those fixtures bit-for-bit (and against the live
-reference when /root/reference exists).
+a reference checkout: `tests/golden/make_golden.py` imports the reference, runs seeded tiny configs of
+all four models and the four nn blocks (and a 3-step Adam trajectory of each model), and commits
+inputs/outputs under tests/golden/; `tests/test_oracle.py` checks this file against those fixtures.
 """
 
 import math

@@ -1,10 +1,11 @@
 """Generates the golden fixtures in this directory by running the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):  python tests/golden/make_golden.py
+Needs a checkout of the reference (EugenHotaj/pytorch-generative):
+    python tests/golden/make_golden.py <path to the pytorch-generative checkout>
 The reference's own tests hold no numeric vectors for this path (SURVEY.md §8c), so these fixtures —
 outputs of the reference itself on seeded inputs — are what pins the oracle (oracle/reference_path.py)
-and, through it, the CUDA path.  Each fixture is a small torch .pt dict; nothing else in the repo reads
-/root/reference at test time on the GPU box.
+and, through it, the CUDA path.  Each fixture is a small torch .pt dict; the tests read only these files,
+never the reference itself.
 
 Fixtures
   model_<name>.pt : cfg, state_dict (default init under manual_seed + N(0, 0.05) noise so that biases,
@@ -16,6 +17,8 @@ Fixtures
                     outputs and all gradients.
   nn_linear_attention.pt : LinearCausalAttention (one head; two heads with embed != out channels): output, all gradients.
   receptive_fields.pt : debug.compute_receptive_field-style 7x7 causality patterns of the four models.
+  adam_trajectory.pt : three recipe training steps of each model from its model_<name>.pt weights: loss and
+                    gradient norm of every step, floating-point state after the last step.
 """
 
 import os
@@ -24,7 +27,6 @@ import warnings
 
 import torch
 
-REF = "/root/reference"
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 MODEL_CFGS = {
@@ -196,10 +198,39 @@ def make_linear_attention_fixture(pg):
     return out
 
 
+def make_adam_trajectory(pg):
+    """Trainer._train_one_batch (reference trainer.py:173-193) three times per model, from the model fixture's weights,
+    on uniform batches drawn from one seeded generator: zero_grad, forward, recipe loss, backward,
+    clip_grad_norm_(1e50), Adam, MultiplicativeLR."""
+    out = {}
+    for name, spec in MODEL_CFGS.items():
+        fx = torch.load(os.path.join(HERE, f"model_{name}.pt"), weights_only=False)
+        model = getattr(pg.models, spec["cls"])(**spec["kwargs"])
+        model.load_state_dict(fx["state_before"])
+        lr = 5e-3 if name == "image_gpt" else 1e-3
+        opt = torch.optim.Adam(model.parameters(), lr=lr)
+        sched = torch.optim.lr_scheduler.MultiplicativeLR(opt, lr_lambda=lambda _: 0.999977)
+        g = torch.Generator().manual_seed(11)
+        losses, norms = [], []
+        for _ in range(3):
+            x = torch.rand(fx["x"].shape, generator=g)
+            opt.zero_grad()
+            loss = loss_fn(x, model(x))
+            loss.backward()
+            norm = torch.nn.utils.clip_grad_norm_(model.parameters(), 1e50)
+            opt.step()
+            sched.step()
+            losses.append(loss.item())
+            norms.append(norm.item())
+        state = {k: v.detach().clone() for k, v in model.state_dict().items() if v.is_floating_point()}
+        out[name] = dict(lr=lr, data_seed=11, losses=losses, norms=norms, state=state)
+    return out
+
+
 def main():
-    if not os.path.isdir(REF):
-        sys.exit("make_golden.py needs the reference checkout at /root/reference")
-    sys.path.insert(0, REF)
+    if len(sys.argv) != 2 or not os.path.isdir(os.path.join(sys.argv[1], "pytorch_generative")):
+        sys.exit("usage: make_golden.py <path to the pytorch-generative checkout>")
+    sys.path.insert(0, os.path.abspath(sys.argv[1]))
     warnings.filterwarnings("ignore")
     torch.set_num_threads(1)  # deterministic summation order for the fixtures
     import pytorch_generative as pg
@@ -213,6 +244,8 @@ def main():
     print("nn_blocks.pt, receptive_fields.pt written")
     torch.save(make_linear_attention_fixture(pg), os.path.join(HERE, "nn_linear_attention.pt"))
     print("nn_linear_attention.pt written")
+    torch.save(make_adam_trajectory(pg), os.path.join(HERE, "adam_trajectory.pt"))
+    print("adam_trajectory.pt written")
 
 
 if __name__ == "__main__":

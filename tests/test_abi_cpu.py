@@ -88,14 +88,37 @@ def test_sample_argument_contract():
         m.sample(n_samples=1)  # before any forward: shape buffers do not exist yet, as in the reference
 
 
-def test_overlay_rebinds_reference_names():
+# Where the reference package (pytorch_generative) defines the names the overlay rebinds: `nn` re-exports them from
+# two modules, `models` from one module per model under the namespace package `models.autoregressive`.
+_REF_LAYOUT = {
+    "nn/attention.py": ["CausalAttention", "LinearCausalAttention", "image_positional_encoding"],
+    "nn/convolution.py": ["CausalConv2d", "GatedActivation", "NCHWLayerNorm"],
+    "models/autoregressive/pixel_cnn.py": ["PixelCNN"],
+    "models/autoregressive/gated_pixel_cnn.py": ["GatedPixelCNN"],
+    "models/autoregressive/pixel_snail.py": ["PixelSNAIL"],
+    "models/autoregressive/image_gpt.py": ["ImageGPT"],
+}
+
+
+def _write_reference_stand_in(root):
+    """A package with the reference's module layout whose names are placeholders (the overlay only rebinds them)."""
+    pkg = root / "pytorch_generative"
+    inits = {"": "from pytorch_generative import models, nn\n", "nn": "", "models": ""}
+    for rel, names in _REF_LAYOUT.items():
+        (pkg / rel).parent.mkdir(parents=True, exist_ok=True)
+        (pkg / rel).write_text("".join(f"class {n}:\n    pass\n" for n in names))
+        mod = "pytorch_generative." + rel[:-3].replace("/", ".")
+        inits[rel.split("/")[0]] += f"from {mod} import {', '.join(names)}\n"
+    for sub, text in inits.items():
+        (pkg / sub / "__init__.py").write_text(text)
+
+
+def test_overlay_rebinds_reference_names(tmp_path):
     """overlay.install() makes the reference package hand out the B200 classes (and uninstall() restores it)."""
-    import os
     import sys
 
-    if not os.path.isdir("/root/reference/pytorch_generative"):
-        pytest.skip("reference checkout not present")
-    sys.path.insert(0, "/root/reference")
+    _write_reference_stand_in(tmp_path)
+    sys.path.insert(0, str(tmp_path))
     try:
         import pytorch_generative as ref
 
@@ -112,8 +135,12 @@ def test_overlay_rebinds_reference_names():
         finally:
             overlay.uninstall()
         assert ref.models.ImageGPT is orig
+        assert ref.models.autoregressive.pixel_snail.PixelSNAIL is not models.PixelSNAIL
+        assert ref.nn.CausalAttention is not nn.CausalAttention
     finally:
-        sys.path.remove("/root/reference")
+        sys.path.remove(str(tmp_path))
+        for name in [n for n in sys.modules if n == "pytorch_generative" or n.startswith("pytorch_generative.")]:
+            del sys.modules[name]
 
 
 def test_ctypes_structs_and_signatures_match_the_header(tmp_path):

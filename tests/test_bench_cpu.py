@@ -21,6 +21,28 @@ def test_reference_arm_prints_one_json_line():
     assert d["e2e"] == {"value": d["value"], "unit": "images/sec", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_dump_outputs_writes_the_step_results_and_a_fixed_weight_sample(tmp_path):
+    import numpy as np
+    import torch
+
+    import bench
+
+    model = torch.nn.Linear(3000, 2)  # weight: 6000 elements, sampled down to per_tensor; bias: kept whole
+    logits = torch.randn(2, 3, 4, 4, dtype=torch.bfloat16)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), (1.25, 3.5), logits, model)
+    assert sorted(os.listdir(tmp_path / "a")) == ["grad_norm.npy", "logits.npy", "loss.npy", "weights.npy"]
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")}
+    assert got["loss"].dtype == got["grad_norm"].dtype == np.float64 and got["loss"] == 1.25 and got["grad_norm"] == 3.5
+    assert got["logits"].dtype == np.float32 and np.array_equal(got["logits"], logits.float().numpy())
+    w = got["weights"]
+    assert w.dtype == np.float32 and w.shape == (4096 + 2,)
+    assert np.isin(w[:4096], model.weight.detach().numpy()).all() and np.array_equal(w[4096:], model.bias.detach().numpy())
+    assert np.array_equal(w, np.load(tmp_path / "b" / "weights.npy"))  # the same positions on every run
+    bench.dump_outputs(str(tmp_path / "c"), (1.25, 3.5), logits, model, max_logits=2 * 3 * 4 * 4 - 1)
+    assert np.array_equal(np.load(tmp_path / "c" / "logits.npy"), logits[:1].float().numpy())  # leading images only
+
+
 def test_reference_arm_is_silent_on_other_ranks():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     proc = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"],
